@@ -23,6 +23,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as it found it (it may be read-only)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -44,6 +45,35 @@ def measured_peak():
             return float(json.load(f)["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
     except Exception:
         return HBM_FALLBACK_GBS, "fallback (B200_PROFILING.md 6.65 TB/s)"
+
+
+# ------------------------------------------------------------------ --dump-outputs
+DUMP_SAMPLE_ROWS = 1 << 19   # rows kept of each large result: 4 MB per float64 array, the whole dump stays far below the limit
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def sample_rows(n):
+    """sorted positions of a fixed, seeded sample of n rows (all of them when n is small): the same rows in every run"""
+    if n <= DUMP_SAMPLE_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(12345).choice(n, DUMP_SAMPLE_ROWS, replace=False))
+
+
+def write_dump(dump_dir, arrays):
+    """one DIR/<name>.npy per array; float32 / float64 only, DUMP_LIMIT_BYTES in all"""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(dump_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if a.dtype not in (np.float32, np.float64):
+            raise TypeError(f"--dump-outputs: {name} is {a.dtype}, not float32 / float64")
+        np.save(os.path.join(dump_dir, name + ".npy"), a)
+
+
+def int64_halves(name, v):
+    """an int64 column float64 cannot hold exactly, as its high (signed) and low 32-bit halves: both exact in float64"""
+    return {name + "_hi32": (v >> 32).astype(np.float64), name + "_lo32": (v & 0xFFFFFFFF).astype(np.float64)}
 
 
 # ------------------------------------------------------------------ synthetic tables (SURVEY §8d)
@@ -161,9 +191,10 @@ class JoinBench:
         self._keep = (t, k)
         return L.TQJoinDesc(0, 1, 2, t, 2, t, 1, k, k, batch, flags)
 
-    def step_device(self, keep=False):
+    def step_device(self, keep=False, hold=False):
         """build + probe with inputs resident in HBM; returns (joined rows, probe kernel ns, build ns).  keep=True copies the
-        four result columns to the host (verification leg, outside every timed region)."""
+        four result columns to the host (verification leg, outside every timed region).  hold=True leaves the handle and the
+        result it lends alive until take_held() (the last timed step of a --dump-outputs run)."""
         L, lib = self.L, self.lib
         h = C.c_void_p()
         d = self.desc()
@@ -184,15 +215,36 @@ class JoinBench:
         st = (C.c_int64 * 8)()
         lib.tq_join_stats(h, st)
         rows = n.value
-        self.last_out = None
-        if keep:
-            self.last_out = []
-            for c in range(4):
-                a = np.empty(rows, dtype=np.int64)
-                L.check(lib.tq_memcpy_d2h(a.ctypes.data, out[c].data, rows * 8))
-                self.last_out.append(a)
-        L.check(lib.tq_join_destroy(h))
+        self.last_out = self._copy_out(out, rows) if keep else None
+        if hold:
+            self.held = (h, out, rows)
+        else:
+            L.check(lib.tq_join_destroy(h))
         return rows, st[5], st[6]
+
+    def _copy_out(self, out, rows):
+        cols = []
+        for c in range(4):
+            a = np.empty(rows, dtype=np.int64)
+            self.L.check(self.lib.tq_memcpy_d2h(a.ctypes.data, out[c].data, rows * 8))
+            cols.append(a)
+        return cols
+
+    def take_held(self):
+        """the result of the held step as --dump-outputs arrays: the rows of a seeded sample of probe rows, in probe-row
+        order (the hash join's output order is not part of its result), plus the row count; then the handle is destroyed"""
+        h, out, rows = self.held
+        self.held = None
+        bk, bv, pkk, pv = self._copy_out(out, rows)
+        self.L.check(self.lib.tq_join_destroy(h))
+        mark = np.zeros(self.n_probe, dtype=bool)
+        mark[sample_rows(self.n_probe)] = True
+        pos = np.flatnonzero(mark[pv])
+        pos = pos[np.argsort(pv[pos], kind="stable")]
+        # every value of C3 is below 2^53 (keys < n_build, B.v = 7k+1, row ids < n_probe): float64 holds it exactly
+        return {"join_rows": np.array([rows], dtype=np.float64), "join_build_key": bk[pos].astype(np.float64),
+                "join_build_value": bv[pos].astype(np.float64), "join_probe_key": pkk[pos].astype(np.float64),
+                "join_probe_value": pv[pos].astype(np.float64)}
 
     def verify(self):
         """Full-size value check of the device-resident join (outside the timed region): output = (B.k, B.v, P.k, P.v)."""
@@ -358,14 +410,16 @@ def run_join_bench(args, rank, world, local_rank, dist):
     probe_ns, build_ns = [], []
     ms = C.c_float(0)
     L.check(lib.tq_timer_start())
-    for _ in range(args.steps):
-        rows, pns, bns = jb.step_device()
+    for i in range(args.steps):
+        rows, pns, bns = jb.step_device(hold=args.dump is not None and i == args.steps - 1)
         probe_ns.append(pns)
         build_ns.append(bns)
     L.check(lib.tq_timer_stop(C.byref(ms)))
     lib.tq_device_synchronize()
     clocks = sampler.stop()
     launches2 = lib.tq_kernel_launch_count()
+    if args.dump is not None:
+        args.dump.update(jb.take_held())
     ms_per_step = ms.value / args.steps
     value = n_probe / (ms_per_step * 1e-3)
     # roofline of the dominant kernels (the probe pipeline): 64 algorithmic bytes per probe row (SURVEY §8d / DESIGN.md)
@@ -421,11 +475,9 @@ def run_secondary(args, lib, peak, peak_src):
     record: value, roofline, cpu_baseline, e2e and a full-size value check each; timed after the headline."""
     import bench_extra
     sec = {}
-    sub = argparse.Namespace(**vars(args))
-    sub.steps, sub.warmup = max(3, min(args.steps, 10)), max(3, min(args.warmup, 5))
     for name, fn in (("C2", bench_extra.run_expr), ("C4", bench_extra.run_agg)):
         try:
-            r = fn(sub, lib, peak, peak_src, ClockSampler)
+            r = fn(args, lib, peak, peak_src, ClockSampler)
             sec[name] = {k: r[k] for k in ("metric", "value", "unit", "ms_per_step", "steps", "warmup", "config", "roofline", "e2e", "cpu_baseline", "verified", "gpu_launches", "clocks")
                          if k in r}
         except Exception as e:  # the headline line must survive a secondary failure; the failure itself is reported
@@ -488,10 +540,18 @@ def main():
     ap.add_argument("--verify", action="store_true", help="with --kernel-only: still run the full-size value check")
     ap.add_argument("--no-secondary", action="store_true", help="skip the C2 / C4 secondary block")
     ap.add_argument("--no-chunked-e2e", action="store_true", help="skip the <=1024-row chunk protocol e2e figure")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step of every workload timed as DIR/<name>.npy (float64, seeded samples "
+                         "of large results, at most 64 MB); that step's handle is released after the timer stops")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl == "reference" or args.gpus > 1 or world > 1):
+        ap.error("--dump-outputs dumps the single-GPU device path (--impl ours, --gpus 1)")
+    args.dump = {} if args.dump_outputs else None
     if args.impl == "reference":
         out = run_reference(args, rank)
         if out is not None:
@@ -509,6 +569,8 @@ def main():
     else:
         import bench_extra
         out = bench_extra.run(args, rank, world, local_rank)
+    if args.dump is not None:
+        write_dump(args.dump_outputs, args.dump)
     if rank == 0 and out is not None:
         print(json.dumps(out))
     if dist is not None:

@@ -11,7 +11,7 @@ import time
 import numpy as np
 
 from tinysql_b200 import _lib as L
-from tinysql_b200.chunk import FLOAT64, INT64, Column, DeviceColumn
+from tinysql_b200.chunk import FLOAT64, INT64, Column, DeviceColumn, device_to_host
 
 
 def _pinned(lib, n_items, dtype, src=None):
@@ -62,6 +62,12 @@ def run_expr(args, lib, peak, peak_src, sampler_cls):
     l1 = lib.tq_kernel_launch_count()
     ms_fused = timed(fused)
     l2 = lib.tq_kernel_launch_count()
+    if args.dump is not None:   # lt / plus hold the last fused step's result until the separate-ops timing overwrites them
+        from bench import int64_halves, sample_rows
+        rows = sample_rows(n)
+        h_lt, h_plus = lt.to_host(), plus.to_host()
+        args.dump["expr_lt"] = h_lt.values[rows].astype(np.float64)
+        args.dump.update(int64_halves("expr_plus", h_plus.values[rows]))
     ms_sep = timed(separate)
     clocks = sampler.stop()
     # e2e: pinned host columns through the host path (slab pipeline: H2D | kernel | D2H overlapped)
@@ -122,7 +128,10 @@ def run_agg(args, lib, peak, peak_src, sampler_cls):
     funcs = (L.TQAggFunc * 3)(L.TQAggFunc(1, 1), L.TQAggFunc(0, -1), L.TQAggFunc(5, 0))  # SUM(x), COUNT(*), firstrow(k)
     desc = L.TQAggDesc(2, types, 1, gb, 3, funcs, groups)
 
-    def step(mem, cols_fn):
+    held = []
+
+    def step(mem, cols_fn, hold=False):
+        """hold=True keeps the handle and the result it lends for the --dump-outputs copy after the timer stops"""
         h = C.c_void_p()
         L.check(lib.tq_agg_create(C.byref(desc), C.byref(h)))
         cols_fn(h)
@@ -132,7 +141,10 @@ def run_agg(args, lib, peak, peak_src, sampler_cls):
         L.check(lib.tq_agg_next_device(h, out, C.byref(nn), C.byref(eof)))
         st = (C.c_int64 * 4)()
         lib.tq_agg_stats(h, st)
-        L.check(lib.tq_agg_destroy(h))
+        if hold:
+            held.append((h, out, nn.value))
+        else:
+            L.check(lib.tq_agg_destroy(h))
         return nn.value, st[2]
 
     def dev_put(h):
@@ -149,12 +161,21 @@ def run_agg(args, lib, peak, peak_src, sampler_cls):
     ms = C.c_float(0)
     upd = []
     L.check(lib.tq_timer_start())
-    for _ in range(args.steps):
-        g, ns = step(L.TQ_MEM_DEVICE, dev_put)
+    for i in range(args.steps):
+        g, ns = step(L.TQ_MEM_DEVICE, dev_put, hold=args.dump is not None and i == args.steps - 1)
         upd.append(ns)
     L.check(lib.tq_timer_stop(C.byref(ms)))
     clocks = sampler.stop()
     l2 = lib.tq_kernel_launch_count()
+    if held:
+        # SUM, COUNT, firstrow(k) of a seeded sample of the groups in key order (the group table's order is not part of the result)
+        from bench import sample_rows
+        h, out, ng = held.pop()
+        res = [device_to_host(tp, out[i].data, None, ng).values for i, tp in enumerate((FLOAT64, INT64, INT64))]
+        L.check(lib.tq_agg_destroy(h))
+        rows = np.argsort(res[2], kind="stable")[sample_rows(ng)]
+        args.dump.update({"agg_groups": np.array([ng], dtype=np.float64), "agg_sum": res[0][rows], "agg_count": res[1][rows].astype(np.float64),
+                          "agg_key": res[2][rows].astype(np.float64)})
     ms_step = ms.value / args.steps
     pk, _ = _pinned(lib, n, np.int64, k)
     px, _ = _pinned(lib, n, np.float64, x)
